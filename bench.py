@@ -87,6 +87,26 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+def host_outputs(results, limit=60 << 20):
+    """{name: float32 array} of the tensors the timed path returned for its last step (one result per lane, the fields of
+    BatchEditResult / MasaCtrlBatchResult / the EDICT latents), at most `limit` bytes in all (under 64 MB with the .npy
+    headers): an array larger than its share of what is left keeps every s-th entry of its first axis (s fixed by the
+    sizes), smaller arrays are kept whole.  The inputs are seeded, so two builds can be compared output for output."""
+    fields = {}
+    for ln, r in enumerate(results):
+        for k, v in vars(r).items():
+            if isinstance(v, torch.Tensor) and v.is_floating_point():
+                fields[k if len(results) == 1 else f"lane{ln}_{k}"] = v
+    out, left = {}, limit
+    for i, (k, v) in enumerate(sorted(fields.items(), key=lambda kv: kv[1].numel())):
+        share = left // (len(fields) - i)
+        stride = -(-v.numel() * 4 // share)
+        a = v.detach()[::stride] if stride > 1 else v.detach()
+        out[k] = a.float().cpu().numpy()
+        left -= out[k].nbytes
+    return out
+
+
 def cpu_unet_times(state_dict, threads, reps=1, which=("b4", "b1")):
     """Times the CPU oracle port (oracle/unet_ref.py, fp32 like the reference's P2P path) on the host cores."""
     from oracle import unet_ref
@@ -191,6 +211,8 @@ def main():
                          "inside every pass")
     ap.add_argument("--lanes", type=int, default=1,
                     help="passes in flight per GPU (own CUDA stream / engine handle / host thread, shared weights)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -305,12 +327,20 @@ def main():
     e0.record()
     outs = []
     for i in range(args.steps):
-        outs.extend(r.latents for r in edit_step([z_pass[first + i * NL + ln] for ln in range(NL)]))
+        last = edit_step([z_pass[first + i * NL + ln] for ln in range(NL)])
+        outs.extend(r.latents for r in last)
     e1.record()
     torch.cuda.synchronize()
     if dist is not None:
         dist.barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        # copied now: the passes measured below may reuse the buffers these results live in
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k, a in host_outputs(last).items():
+            np.save(os.path.join(args.dump_outputs, f"{k}.npy"), a)
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if dist is not None:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)

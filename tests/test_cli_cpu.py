@@ -1,5 +1,6 @@
 """The `run_editing_*` entry-point plumbing on the CPU: dataset schema, RLE mask decoding (against the reference's own
-function where the tree is mounted), output layout, skip-if-exists, and the image-parallel split of the work list."""
+function, recorded in tests/golden/reference_cli.npz), output layout, skip-if-exists, and the image-parallel split of the
+work list."""
 import ast
 import json
 import os
@@ -9,12 +10,14 @@ import pytest
 
 from pnpinversion_b200 import cli
 from pnpinversion_b200.parallel import shard_sizes
+from oracle import ref_shim
+from tests.reference_golden import recorded_fixture
 
-REF = os.environ.get("PNP_REFERENCE_ROOT", "/root/reference")
+golden = recorded_fixture("cli")
 
 
 def _reference_mask_decode():
-    path = os.path.join(REF, "run_editing_p2p.py")
+    path = os.path.join(ref_shim.REF, "run_editing_p2p.py")
     with open(path) as f:
         tree = ast.parse(f.read(), filename=path)
     tree.body = [n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == "mask_decode"]
@@ -23,18 +26,17 @@ def _reference_mask_decode():
     return ns["mask_decode"]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted")
-def test_mask_decode_matches_the_reference_function():
-    ref = _reference_mask_decode()
+def test_mask_decode_matches_the_reference_function(golden):
+    ref = _reference_mask_decode() if golden.recording else None
     rng = np.random.RandomState(0)
-    for _ in range(5):
+    for i in range(5):
         starts = np.sort(rng.choice(512 * 512 - 600, size=40, replace=False))
         rle = []
         for s in starts:
             rle += [int(s), int(rng.randint(1, 500))]
         rle += [512 * 512 - 10, 500]  # a run that overshoots the image: clipped (run_editing_p2p.py:16)
-        assert np.array_equal(cli.mask_decode(rle), ref(rle))
-    assert np.array_equal(cli.mask_decode([]), ref([]))
+        assert golden.equal(f"mask_decode/{i}", cli.mask_decode(rle), lambda: ref(rle))
+    assert golden.equal("mask_decode/empty", cli.mask_decode([]), lambda: ref([]))
 
 
 def test_mask_round_trip_and_border():
